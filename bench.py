@@ -261,6 +261,19 @@ def check_q5(gpu_rows, cpu_rows):
     return all(g[0] == c[0] and _close(g[1], c[1]) for g, c in zip(gpu_rows, cpu_rows))
 
 
+def dump_outputs(out_dir, results):
+    """results: leg -> pyarrow.Table.  One float64 array per column (dates as days since the epoch, NULL as NaN); the query
+    results are at most a few dozen rows, far below any size worth sampling."""
+    import pyarrow as pa
+    os.makedirs(out_dir, exist_ok=True)
+    for leg, tbl in results.items():
+        for name in tbl.column_names:
+            col = tbl.column(name)
+            if pa.types.is_date(col.type):
+                col = col.cast(pa.int32())
+            np.save(os.path.join(out_dir, "%s_%s.npy" % (leg, name)), col.cast(pa.float64()).to_numpy())
+
+
 def run_reference(args, rank):
     """--impl reference: the reference's CPU path (oracle port) on the same rows, host cores only; rank 0 alone works."""
     if rank != 0:
@@ -316,6 +329,8 @@ def main():
     ap.add_argument("--no-verify", action="store_true")
     ap.add_argument("--profile-host", action="store_true", help="cProfile one untimed step of every join leg to stderr (debugging)")
     ap.add_argument("--config", action="append", default=[], metavar="KEY=VALUE", help="sb_config_set(KEY, VALUE) before the run (A/B experiments)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the result of the last timed step of every query leg to DIR/<leg>_<column>.npy "
+                                                          "(float64), to compare two builds output for output")
     args = ap.parse_args()
     args.legs = [x for x in args.legs.split(",") if x]
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
@@ -478,6 +493,20 @@ def main():
 
     legs = {}
     cpu_info = None
+    # A timed step keeps the batch it returns until the leg's next step starts (the same one release per step as closing it at
+    # once), so the last timed step's result is still there for --dump-outputs.
+    held = {}
+    results = {}
+
+    def release_held(leg):
+        b = held.pop(leg, None)
+        if b is not None:
+            b.close()
+
+    def take_result(leg):
+        if args.dump_outputs:
+            results[leg] = held[leg].to_arrow(stream)
+        release_held(leg)
 
     def cpu_leg(leg):
         """Oracle answer for this rank's shard (verification) and, at N = 1 on rank 0, the timed CPU baseline."""
@@ -516,10 +545,11 @@ def main():
             return out
 
         def step_q1():
-            out = q1_plan.executeColumnar(stream)
-            out.close()
+            release_held("q1")
+            held["q1"] = q1_plan.executeColumnar(stream)
 
         ms, launches, prof = time_resident(step_q1, args.steps, args.warmup, ("agg_update",))
+        take_result("q1")
         plan_name = lib.sb_hash_aggregate_last_plan().decode()
         # which kernels ran the big launch: run the Partial stage once more and ask
         p_once = partial.executeColumnar(stream); p_once.close()
@@ -540,6 +570,7 @@ def main():
         capi.config_set("agg_rtc", 0)
         v_ms, _, v_prof = time_resident(step_q1, max(3, args.steps // 4), 1, ("agg_update",))
         variants["generic_kernels"] = {"ms_per_step": v_ms, "agg_update_ms": v_prof["agg_update"][0] / max(1, max(3, args.steps // 4))}
+        release_held("q1")
         capi.config_set("agg_rtc", 1)
         # the same query over NULLable columns handed over in another order (what a Parquet scan of a nullable schema gives Spark).
         # (a) the batch declares null_count = 0 (ColumnVector.hasNull() == false): the bitmaps are never read, same kernels as the
@@ -625,8 +656,8 @@ def main():
         local_plan, merged_plan = build(src)
 
         def step_join():
-            out = merged_plan.executeColumnar(stream)
-            out.close()
+            release_held(leg)
+            held[leg] = merged_plan.executeColumnar(stream)
 
         steps = max(1, min(args.steps, args.leg_steps))
         if args.profile_host and rank == 0:
@@ -640,6 +671,7 @@ def main():
             pr.disable()
             pstats.Stats(pr, stream=sys.stderr).sort_stats("cumulative").print_stats(25)
         ms, launches, prof = time_resident(step_join, steps, max(3, args.warmup), ("join_build", "join_probe", "join_fill", "gather", "filter_project", "agg_update"))
+        take_result(leg)
         alg_bytes = sum(tpch.synth_rows(t, n_orders) * sum(tpch.synth_width(c) for c in cols) for t, cols in used.items())
         achieved = alg_bytes / (ms / 1000.0) / 1e9
         verified = None
@@ -709,6 +741,8 @@ def main():
                            "dataset": "include/sb_synth.h, seed 42 + rank, generated on the device"},
                 "roofline": head.get("roofline"), "cpu_baseline": cpu_info, "e2e": head.get("e2e"), "verified": all(l.get("verified") is not False for l in legs.values()) and any(l.get("verified") for l in legs.values()),
                 "gpu_launches": int(sum(l.get("gpu_launches", 0) for l in legs.values())), "legs": legs, "clocks": clocks}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, results)
         print(json.dumps(line), flush=True)
     for b in tables.values():
         b.close()
